@@ -3,7 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload cfg2|distB|incoherent|cfg3|cfg5] [--scaling weak|strong|frame]
-                    [--exchange fused|nccl] [--lag L] [--grid-storage fp32|bf16]
+                    [--exchange fused|nccl] [--lag L] [--grid-storage fp32|bf16] [--dump-outputs DIR]
 
 Workloads (SURVEY.md 8d; fields built by the reference's constructor defaults, random init):
   cfg2        (default, the headline) one TensorVMSplit at 300^3, seed 0, an 800x800 pinhole frame at
@@ -27,9 +27,9 @@ field: ray generation + march + shading + composite + blend).  Steps walk throug
             ray; samples counted exactly by the kernel) / event-timed launch duration, against the
             measured HBM copy bandwidth in MEASURED_PEAKS.json; `traffic` = DRAM bytes per launch of
             the committed ncu capture of this workload (profiles/traffic.json), or null.
-  cpu_baseline / --impl reference: the UNMODIFIED PyTorch reference (staged byte-identical under
-            baseline/_ref by oracle/vendor_ref.py) on all host cores, 4096 rays per step; the CPU
-            oracle port (oracle/lrf_oracle.c) only if the reference cannot be imported.
+  cpu_baseline / --impl reference: the UNMODIFIED PyTorch reference (its bytecode, compiled by build() into
+            oracle/_ref, or a checkout named by $LOCALRF_REFERENCE; oracle/ref_loader.py) on all host cores,
+            4096 rays per step; the CPU oracle port (oracle/lrf_oracle.c) if neither is there.
             `reference_gpu` = the same unmodified reference with device="cuda" on this B200.
 
 N > 1 (torchrun, one rank per GPU), field replicated, rays sharded, no data-path collective:
@@ -42,6 +42,10 @@ N > 1 (torchrun, one rank per GPU), field replicated, rays sharded, no data-path
   the next launches wait (in their prologue) for the peers' step s-1-lag -- no barrier launch, no collective
   (--exchange fused, --lag 3 default; --lag 0 = same-step barrier kernel); --exchange nccl uses one
   ncclAllGather per step instead.
+
+--dump-outputs DIR: after the timed steps, the arrays the last timed step returned to its caller (rgb, depth,
+  directions, ij of LocalTensorfs.forward; rank 0) are written as DIR/<name>.npy in float32 / float64, so two
+  builds can be compared output for output: the same arguments give the same inputs.
 
 --grid-storage bf16 (NOT the headline; a separate, labelled line): eval kernels gather bfloat16 copies of the
   grids (LocalTensorfs.set_grid_storage); the roofline then counts 288 / 864 B per density / appearance sample.
@@ -318,7 +322,7 @@ def oracle_batch(lt, field, ids, n_threads=None):
 
 
 def load_reference_classes():
-    """The unmodified reference's LocalTensorfs (baseline/_ref or /root/reference), or None."""
+    """The unmodified reference's LocalTensorfs (oracle/ref_loader.py), or None."""
     try:
         from oracle.ref_loader import load_reference, reference_available
         if not reference_available():
@@ -389,7 +393,7 @@ def cpu_baseline(wl, budget_s=20.0):
         dt = time.perf_counter() - t0
         return {"value": BATCH * steps / dt, "unit": "rays/s", "cores": torch.get_num_threads(), "kind": "reference",
                 "sample": f"{steps} batches of 4096 rays of workload {wl.name}, unmodified PyTorch reference "
-                          f"(baseline/_ref, LocalTensorfs.forward, torch {torch.__version__}, "
+                          f"(LocalTensorfs.forward, torch {torch.__version__}, "
                           f"{torch.get_num_threads()} threads), {dt:.2f} s"}
     except Exception as e:
         print(f"bench: reference CPU baseline unavailable ({e}); using the oracle port", file=sys.stderr)
@@ -418,7 +422,7 @@ def run_reference(args):
     kind, cores = "reference", torch.get_num_threads()
     try:
         value, dt = time_reference(wl, "cpu", args.warmup, args.steps)
-        sample = (f"4096 rays per step, unmodified PyTorch reference (baseline/_ref), LocalTensorfs.forward, "
+        sample = (f"4096 rays per step, unmodified PyTorch reference, LocalTensorfs.forward, "
                   f"torch {torch.__version__}, {cores} threads")
     except Exception as e:
         print(f"bench: reference unavailable ({e}); timing the oracle port", file=sys.stderr)
@@ -453,6 +457,17 @@ def run_reference(args):
 
 
 # ---- our arm ---------------------------------------------------------------------------------------
+OUTPUT_NAMES = ("rgb", "depth", "directions", "ij")          # LocalTensorfs.forward's return, in order
+
+
+def dump_outputs(path, outputs):
+    """DIR/<name>.npy of every array a step returned: floating point as float32, integers as float64 (exact)."""
+    os.makedirs(path, exist_ok=True)
+    for name, t in zip(OUTPUT_NAMES, outputs):
+        a = t.detach().cpu().numpy()
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float32 if a.dtype.kind == "f" else np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -473,7 +488,13 @@ def main():
                          "set_grid_storage): fp32 = the parameters (the headline, the reference's precision); "
                          "bf16 = bfloat16 copies, half the gather bytes (a separate, labelled line -- it renders "
                          "the bf16-rounded field)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the arrays the last timed step returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     quiet_stdout()
     if args.steps is None:
         args.steps = 20 if args.impl == "reference" else 157
@@ -572,12 +593,15 @@ def main():
     for i in range(args.steps):
         flush.zero_(); flush.zero_()         # L2 flush between timed iterations (outside the events)
         ev[i][0].record()
-        step(args.warmup + i, ids_dev)
+        last = step(args.warmup + i, ids_dev)
         ev[i][1].record()
     torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
     sampler.stop_flag = True
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+    del last
     times_ms = [a.elapsed_time(c) for a, c in ev]
     total_ms = torch.tensor([sum(times_ms)], device=dev, dtype=torch.float64)
     if world > 1:
@@ -712,7 +736,7 @@ def main():
                 del flush
                 torch.cuda.empty_cache()
                 v, dt = time_reference(wl, dev, 2, 5)
-                ref_gpu = {"value": v, "unit": "rays/s", "what": "the unmodified PyTorch reference (baseline/_ref), "
+                ref_gpu = {"value": v, "unit": "rays/s", "what": "the unmodified PyTorch reference, "
                            f"device=cuda on this GPU, same workload, 5 batches of 4096 rays after 2 warm-ups, {dt:.3f} s"}
             except Exception as e:
                 ref_gpu = {"unavailable": str(e)[:200]}

@@ -1,8 +1,8 @@
 """Generate the golden fixtures by running the UNMODIFIED reference on CPU.
 
-Run in the build container only (needs /root/reference):
+Needs a checkout of facebookresearch/localrf (commit 3905e39); nothing else does:
 
-    python tests/golden/make_golden.py
+    LOCALRF_REFERENCE=<checkout> python tests/golden/make_golden.py [fullsize | sched | vs_reference]
 
 Writes tests/golden/*.npz.  Each file holds the inputs (field parameters in the reference's
 state_dict layout, rays or ray ids, the sample table z actually used) and the reference's outputs.
@@ -21,7 +21,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-sys.path.insert(0, ROOT)
+sys.path[:0] = [ROOT, os.path.dirname(HERE)]
 from oracle.ref_loader import load_reference  # noqa: E402
 
 TensorVMSplit, AlphaGridMask, LocalTensorfs, ray_utils = load_reference()
@@ -455,9 +455,92 @@ def gen_sched():
     save("sched_nc", **arrays)
 
 
+# ---- G10: the bench's workloads through the reference (tests/test_gpu_vs_reference.py, test_gpu_bf16.py,
+# test_bench_workloads.py).  Scenes are rebuilt from their seeds by bench.Workload; stored are the digests of
+# the reference's scenes and, of each compared batch, a fixed seeded sample of SAMPLE_RAYS rays followed by
+# every other ray within TIE_MARGIN of the w > 1e-3 switch (so the test counts the batch's threshold ties
+# exactly); directions / ij of the sample only.
+VS_BATCHES = {"cfg2": (3, 90), "distB": (50,), "incoherent": (0, 7), "cfg3": (60,)}
+SAMPLE_RAYS = 512
+WEIGHT_ROWS = 64
+
+
+def ray_sample(margin, seed):
+    from helpers import TIE_MARGIN
+    s = np.sort(np.random.default_rng(seed).choice(len(margin), SAMPLE_RAYS, replace=False))
+    return np.concatenate([s, np.setdiff1d(np.nonzero(margin < TIE_MARGIN)[0], s)]).astype(np.int16)
+
+
+def gen_vs_reference():
+    import json
+    import bench
+    from helpers import state_digest
+    scenes = {"grid12": {}, "full": {}}
+    for name in ("cfg2", "distB", "incoherent", "cfg3", "cfg5"):
+        scenes["grid12"][name] = state_digest(bench.Workload(name, 12).build(LocalTensorfs, quiet=True).state_dict())
+    arrays = {}
+    for name, batches in VS_BATCHES.items():
+        wl = bench.Workload(name)
+        lt = wl.build(LocalTensorfs, quiet=True)
+        scenes["full"][name] = state_digest(lt.state_dict())
+        ids, views = wl.batches()
+        kw = wl.call_kwargs(lt, torch.device("cpu"))
+        n_f = len(lt.tensorfs)
+        for b in batches:
+            _captured.clear()
+            _captured["keep_margins"] = True
+            with torch.no_grad():
+                rgb, depth, dirs, ij = quiet(lt, ids[b], views[b], 800, 800, **kw)
+            m = _captured["margins"]                  # alpha2weights calls arrive chunk-major, field-minor
+            margin = torch.stack([torch.cat(m[k::n_f]) for k in range(n_f)]).min(0).values.numpy()
+            s = ray_sample(margin, b)
+            p = f"{name}.b{b}."
+            arrays.update({p + "rays": s, p + "rgb": rgb.numpy()[s], p + "depth": depth.numpy()[s],
+                           p + "margin": margin[s], p + "directions": dirs.numpy()[s[:SAMPLE_RAYS]],
+                           p + "ij": ij.numpy()[s[:SAMPLE_RAYS]].astype(np.int16)})
+        if name != "cfg2":
+            continue
+        # per-sample weights of one field, random rays (white background, the field's own forward)
+        g = torch.Generator().manual_seed(4)
+        rays = torch.cat([0.1 * torch.randn(4096, 3, generator=g), torch.randn(4096, 3, generator=g)], -1)
+        _captured.clear()
+        with torch.no_grad():
+            rgb, depth = lt.tensorfs[0](rays, is_train=False, white_bg=True, N_samples=-1)
+        w = _captured["weights"].numpy()
+        margin = np.abs(w - 1e-3).min(-1)
+        s = ray_sample(margin, 4)
+        arrays.update({"weights.rays": s, "weights.rgb": rgb.numpy()[s], "weights.depth": depth.numpy()[s],
+                       "weights.margin": margin[s], "weights.rows": s[:WEIGHT_ROWS], "weights.w": w[s[:WEIGHT_ROWS]]})
+        # batch 77 with every plane / line rounded to bfloat16 (the bf16 grid-storage test's field)
+        with torch.no_grad():
+            for rf in lt.tensorfs:
+                for plist in (rf.density_plane, rf.density_line, rf.app_plane, rf.app_line):
+                    for q in plist:
+                        q.copy_(q.to(torch.bfloat16).to(torch.float32))
+        _captured.clear()
+        _captured["keep_margins"] = True
+        with torch.no_grad():
+            rgb, depth, _, _ = quiet(lt, ids[77], views[77], 800, 800, **kw)
+        margin = torch.cat(_captured["margins"]).numpy()
+        s = ray_sample(margin, 77)
+        arrays.update({"bf16.b77.rays": s, "bf16.b77.rgb": rgb.numpy()[s], "bf16.b77.depth": depth.numpy()[s],
+                       "bf16.b77.margin": margin[s]})
+    path = os.path.join(HERE, "vs_reference.npz")
+    np.savez_compressed(path, meta=np.array(META), **arrays)
+    print(f"vs_reference: {os.path.getsize(path) / 1e6:.2f} MB")
+    with open(os.path.join(HERE, "bench_scenes.json"), "w") as f:
+        json.dump({"meta": META, "what": "state_dict digests (tests/helpers.py state_digest) of the reference's "
+                   "scenes built by bench.Workload; grid12 at a 12^3 grid, full at the workload's own size",
+                   **scenes}, f, indent=1)
+        f.write("\n")
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "fullsize":
         gen_fullsize()
+        sys.exit(0)
+    if len(sys.argv) > 1 and sys.argv[1] == "vs_reference":
+        gen_vs_reference()
         sys.exit(0)
     if len(sys.argv) > 1 and sys.argv[1] == "sched":
         gen_sched()

@@ -44,6 +44,18 @@ def full_field_dict(g, prefix=""):
     return fd
 
 
+def state_digest(sd):
+    """sha256 of a state_dict's keys, order, dtypes, shapes and bytes: equal digests <=> equal state_dicts,
+    so a scene can be compared with one that is not at hand."""
+    import hashlib
+    h = hashlib.sha256()
+    for k, v in sd.items():
+        a = np.ascontiguousarray(v.detach().cpu().numpy())
+        h.update(f"{k}|{a.dtype.str}|{a.shape}|".encode())
+        h.update(a.tobytes())
+    return h.hexdigest()
+
+
 def rel_err(a, b, floor=1e-3):
     """max |a-b| / max(|b|, floor): the parity metric (1e-4 relative, fp32)."""
     a = np.asarray(a, dtype=np.float64); b = np.asarray(b, dtype=np.float64)
@@ -72,9 +84,10 @@ def ray_err(a, b, floor=1e-3):
     return np.max(np.abs(a - b) / np.maximum(np.abs(b), floor), axis=1)
 
 
-def check_with_ties(out, ref, margin, tol=1e-4, what="", max_tie_frac=0.01):
+def check_with_ties(out, ref, margin, tol=1e-4, what="", max_tie_frac=0.01, n_total=None):
     """Every ray within `tol` of the reference, except proven threshold ties.  Returns
-    (n_ties, worst error among the non-tie rays)."""
+    (n_ties, worst error among the non-tie rays).  `n_total`: the rays are a subset of a batch of that many
+    that holds every ray with margin < TIE_MARGIN, so the ties counted are all of the batch's."""
     err = ray_err(out, ref)
     bad = np.nonzero(err > tol)[0]
     margin = np.asarray(margin, np.float64)
@@ -82,6 +95,7 @@ def check_with_ties(out, ref, margin, tol=1e-4, what="", max_tie_frac=0.01):
                    if not (margin[r] < TIE_MARGIN and err[r] < TIE_MAX_ERR)]
     assert not unexplained, (f"{what}: {len(unexplained)} rays beyond {tol} that are NOT threshold ties "
                              f"(ray, err, min|w-thres|): {unexplained[:8]}")
-    assert len(bad) <= max_tie_frac * len(err), f"{what}: {len(bad)} threshold ties of {len(err)} rays"
+    n_total = len(err) if n_total is None else n_total
+    assert len(bad) <= max_tie_frac * n_total, f"{what}: {len(bad)} threshold ties of {n_total} rays"
     ok = np.ones(len(err), bool); ok[bad] = False
     return len(bad), float(err[ok].max()) if ok.any() else 0.0

@@ -1,30 +1,23 @@
 """CPU-only: the bench's workloads build IDENTICAL scenes through the product's constructors and through the
 unmodified reference's (same RNG consumption, same append_frame / append_rf bookkeeping), so `bench.py`'s two arms
-and `reference_gpu` render the same thing; batches have the advertised shapes.  Small grids; skipped when no
-reference copy (/root/reference or baseline/_ref) is available."""
+and `reference_gpu` render the same thing; batches have the advertised shapes.  Small grids; the reference's scenes
+are pinned by their state_dict digests (tests/golden/bench_scenes.json, tests/golden/make_golden.py)."""
+import json
+import os
+
 import pytest
 import torch
 
 import bench
-
-
-@pytest.fixture(scope="module")
-def ref_cls():
-    cls = bench.load_reference_classes()
-    if cls is None:
-        pytest.skip("no reference copy available")
-    return cls
+from helpers import GOLDEN, state_digest
 
 
 @pytest.mark.parametrize("name", ["cfg2", "distB", "incoherent", "cfg3", "cfg5"])
-def test_workload_scene_equal_for_product_and_reference(ref_cls, name):
+def test_workload_scene_equal_for_product_and_reference(name):
     import localrf_b200 as L
     wl = bench.Workload(name, 12)
-    ours, ref = wl.build(L.LocalTensorfs, quiet=True), wl.build(ref_cls, quiet=True)
-    sd_o, sd_r = ours.state_dict(), ref.state_dict()
-    assert list(sd_o) == list(sd_r)
-    for k in sd_o:
-        assert torch.equal(sd_o[k], sd_r[k]), k
+    ours = wl.build(L.LocalTensorfs, quiet=True)
+    assert state_digest(ours.state_dict()) == json.load(open(os.path.join(GOLDEN, "bench_scenes.json")))["grid12"][name]
     assert len(ours.tensorfs) == {"cfg3": 3, "cfg5": 8}.get(name, 1)
     assert float(ours.tensorfs[0].density_shift) == (2 if name == "distB" else -5)
     ids, views = wl.batches()
@@ -39,9 +32,12 @@ def test_workload_scene_equal_for_product_and_reference(ref_cls, name):
         assert int((bw > 0).sum(1).max()) == 2 and int((bw > 0).sum(1).min()) == 1
 
 
-def test_reference_arm_line_shape(ref_cls, monkeypatch, capsys):
-    """`--impl reference` prints the contract's JSON keys (tiny grid, 1 step)."""
-    import json, sys
+def test_reference_arm_line_shape(monkeypatch, capsys):
+    """`--impl reference` prints the contract's JSON keys (tiny grid, 1 step).  It times the reference's own
+    code: the bytecode build() compiled into oracle/_ref, or a checkout named by $LOCALRF_REFERENCE."""
+    if bench.load_reference_classes() is None:
+        pytest.skip("no reference (oracle/_ref or $LOCALRF_REFERENCE)")
+    import sys
     monkeypatch.setattr(bench, "_REAL_STDOUT", None)
     monkeypatch.setattr(bench, "quiet_stdout", lambda: None)
     monkeypatch.setattr(sys, "argv", ["bench.py", "--impl", "reference", "--steps", "1", "--warmup", "0", "--grid", "16"])

@@ -8,6 +8,8 @@ fp32-storage render (same arithmetic, same order), and therefore holds the same 
 oracle / the unmodified reference evaluated on those parameters.  On arbitrary parameters the
 bf16-storage render is the fp32 render of the rounded field."""
 import ctypes as C
+import json
+import os
 
 import numpy as np
 import pytest
@@ -16,7 +18,7 @@ import torch
 import localrf_b200 as L
 from localrf_b200 import _lib
 from gpu_helpers import module_from_golden, oracle_fields
-from helpers import check_with_ties, load_golden, rel_err
+from helpers import GOLDEN, check_with_ties, load_golden, rel_err, state_digest
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-4
@@ -143,10 +145,13 @@ def test_bf16_with_positional_encodings_is_refused():
 
 def test_local_tensorfs_bf16_plan_path_and_whole_batch_vs_reference():
     """cfg2 at the BASELINE size: LocalTensorfs eval (plan fast path) from bf16 grids against (a) the fp32
-    storage of the same rounded field and (b) the UNMODIFIED reference on this GPU with the rounded parameters."""
+    storage of the same rounded field and (b) the UNMODIFIED reference's committed outputs with the rounded parameters."""
     import bench
     wl = bench.Workload("cfg2")
-    ours = wl.build(L.LocalTensorfs, quiet=True).to("cuda")
+    ours = wl.build(L.LocalTensorfs, quiet=True)
+    scenes = json.load(open(os.path.join(GOLDEN, "bench_scenes.json")))
+    assert state_digest(ours.state_dict()) == scenes["full"]["cfg2"]      # the reference's scene, before rounding
+    ours = ours.to("cuda")
     for rf in ours.tensorfs:
         round_grids_to_bf16(rf)
     ids, views = wl.batches()
@@ -166,32 +171,12 @@ def test_local_tensorfs_bf16_plan_path_and_whole_batch_vs_reference():
           f"bit-equal: {torch.equal(rgb16, rgb32)})")
     assert e_dep < 1e-5 and n_bad <= 4          # (a flipped w > 1e-3 decision needs a last-bit difference: none expected)
 
-    from oracle.ref_loader import reference_available
-    if not reference_available():
-        pytest.skip("no staged reference (baseline/_ref) on this box")
-    import contextlib, io
-    ref = bench.ReferenceRunner(wl, "cuda")
-    for rf in ref.lt.tensorfs:
-        round_grids_to_bf16(rf)
-    for pa, pb in zip(grids(ref.lt.tensorfs[0]), grids(ours.tensorfs[0])):
-        assert torch.equal(pa, pb)
-    import models.tensorBase as ref_tb
-    cap, orig = [], ref_tb.alpha2weights
-
-    def a2w(alpha):
-        wts, T = orig(alpha)
-        cap.append(wts.detach())
-        return wts, T
-
-    ref_tb.alpha2weights = a2w
-    try:
-        with torch.no_grad(), contextlib.redirect_stdout(io.StringIO()):
-            r_rgb, r_dep, _, _ = ref.lt(ref.ids[b], ref.views[b], 800, 800, **ref.kw)
-    finally:
-        ref_tb.alpha2weights = orig
-    margin = (torch.cat(cap) - 1e-3).abs().min(-1).values.cpu().numpy()
-    n1, e1 = check_with_ties(rgb16.cpu().numpy(), r_rgb.cpu().numpy(), margin, TOL, "cfg2 bf16 storage vs reference rgb")
-    n2, e2 = check_with_ties(dep16.cpu().numpy(), r_dep.cpu().numpy(), margin, TOL, "cfg2 bf16 storage vs reference depth")
-    print(f"cfg2 batch {b}, bf16 grid storage vs the reference on this GPU (rounded parameters): rgb worst {e1:.2e} "
-          f"({n1} threshold ties of 4096), depth worst {e2:.2e}")
+    g = load_golden("vs_reference")             # the reference on the same rounded field (tests/golden/make_golden.py)
+    s, margin = g["bf16.b77.rays"].astype(np.int64), g["bf16.b77.margin"]
+    n1, e1 = check_with_ties(rgb16.cpu().numpy()[s], g["bf16.b77.rgb"], margin, TOL, "cfg2 bf16 storage vs reference rgb",
+                             n_total=4096)
+    n2, e2 = check_with_ties(dep16.cpu().numpy()[s], g["bf16.b77.depth"], margin, TOL,
+                             "cfg2 bf16 storage vs reference depth", n_total=4096)
+    print(f"cfg2 batch {b}, bf16 grid storage vs the reference (rounded parameters): rgb worst {e1:.2e} "
+          f"({n1} threshold ties of 4096, {len(s)} compared), depth worst {e2:.2e}")
     assert n2 == 0

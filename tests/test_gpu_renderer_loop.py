@@ -3,7 +3,8 @@ executed on top of dropin/: its imports `local_tensorfs` / `models.*` resolve to
 (`utils.utils`: visualize_depth etc.) is the reference's own code.  File / plot I/O is stubbed (no savePath,
 draw_poses replaced: it needs matplotlib).  The frames it returns must equal direct forward calls.
 Runs in a subprocess because the reference uses top-level module names (`utils`, `models`).
-Skipped when the staged reference copy (baseline/_ref) is absent."""
+It executes the reference's own renderer module: the bytecode build() compiled into oracle/_ref, or a checkout
+named by $LOCALRF_REFERENCE (the repository holds no reference source)."""
 import os
 import subprocess
 import sys
@@ -59,8 +60,9 @@ print("RENDER_LOOP_OK", len(rgb_maps))
 
 
 def test_reference_renderer_loop_runs_on_dropin():
-    ref = os.path.join(ROOT, "baseline", "_ref", "localTensoRF")
-    if not os.path.isfile(os.path.join(ref, "renderer.py")):
-        pytest.skip("no staged reference (baseline/_ref) on this box")
+    from oracle import ref_loader
+    if not ref_loader.reference_available():
+        pytest.skip("no reference (oracle/_ref or $LOCALRF_REFERENCE)")
+    ref = ref_loader.REF_PKG
     out = subprocess.run([sys.executable, "-c", SCRIPT, ROOT, ref], capture_output=True, text=True, timeout=900)
     assert out.returncode == 0 and "RENDER_LOOP_OK 12" in out.stdout, (out.stdout[-1500:], out.stderr[-3000:])
